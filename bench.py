@@ -7,7 +7,7 @@ A "step" = one forward of the fusion layer over one batch of synthetic (ref, src
 ms_per_step = forward ms.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--workload cfg2|cfg3|cfg4|cfg4_256|sweep] [--exchange peer|p2p|allgather]
+                  [--workload cfg2|cfg3|cfg4|cfg4_256|sweep] [--exchange peer|p2p|allgather] [--dump-outputs DIR]
 
 N>1 (torchrun, one rank per GPU = one camera view per GPU): every rank owns `pairs_per_gpu` frames of its view, the ranks
 exchange feature maps inside the timed region (ViewParallelFusion: peer-mapped reads over NVLink, NCCL send/recv, or NCCL
@@ -16,6 +16,10 @@ all-gather) and every rank fuses its view against its nearest-neighbour view.  W
 `--impl reference` times the reference's own CPU op sequence (oracle/torch_port.py, same ATen operators incl. its torch
 geometry) on the host cores with the same config / steps / warmup keys; the N=1 line of our arm also carries `cpu_baseline`
 (bounded sample of that) and `gpu_reference` (the same op sequence on the same B200: BASELINE.md B2, the >=10x target's denominator).
+
+`--dump-outputs DIR` writes what the last timed step returned (the module's out / corr_pos / attn, and sample_locs when the
+config emits them; rank 0's at N>1; the last K x C shape's for the sweep) as DIR/<name>.npy.  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -46,6 +50,8 @@ WORKLOADS = {
 SWEEP_K, SWEEP_C = (16, 32, 64, 128), (64, 128, 256, 512)
 L2_BYTES = 126 * 1024 * 1024
 METRIC = "epipolar_fusion_forward_views_per_sec"
+OUTPUT_NAMES = ("out", "corr_pos", "attn", "sample_locs")          # the 4-tuple Epipolar.forward returns
+DUMP_BYTES = 64 * 10 ** 6                                          # --dump-outputs writes at most this much in all
 
 
 def algorithmic_bytes(N, C, H, W, K, attn=True, corr=True):
@@ -56,6 +62,20 @@ def algorithmic_bytes(N, C, H, W, K, attn=True, corr=True):
     if corr:
         b += 8 * N * H * W
     return b
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each output tensor as <out_dir>/<name>.npy in float32.  When they add up to more than DUMP_BYTES, each is cut
+    to its share by a fixed, seeded sample of its flattened elements (sorted flat indices), so that runs with the same
+    arguments write the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in zip(OUTPUT_NAMES, outputs) if v is not None}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = int(a.size * (DUMP_BYTES - 4096) / total)                 # 4096: room for the .npy headers
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, size=keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def measured_peaks():
@@ -263,7 +283,7 @@ def run_sweep(args):
     peak, peak_src = measured_peaks()
     rows = []
     N, H, W = 4, 64, 64
-    steps, warmup = min(args.steps, 30), max(3, min(args.warmup, 10))
+    steps, warmup = args.steps, max(3, min(args.warmup, 10))
     for K in SWEEP_K:
         for C in SWEEP_C:
             cfg = epi.make_cfg(KEYPOINT=dict(HEATMAP_SIZE=(H, W), NFEATS=C), EPIPOLAR=dict(SAMPLESIZE=K, USE_CORRECT_NORMALIZE=True))
@@ -279,8 +299,9 @@ def run_sweep(args):
                 torch.cuda.synchronize()
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-                for i in range(steps):
+                for i in range(steps - 1):
                     m(refs[i % n_sets], srcs[i % n_sets], P1, P2)
+                last = m(refs[(steps - 1) % n_sets], srcs[(steps - 1) % n_sets], P1, P2)
                 e1.record(); torch.cuda.synchronize()
                 ms = e0.elapsed_time(e1) / steps
                 lib.epi_kernel_timing_enable(1)
@@ -294,6 +315,8 @@ def run_sweep(args):
             rows.append({"K": K, "C": C, "ms_per_step": ms, "views_per_s": N / (ms * 1e-3), "kernel_ms": kms,
                          "achieved_gbs": balg / (kms * 1e-3) / 1e9, "frac": balg / (kms * 1e-3) / 1e9 / peak})
             del refs, srcs, m
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     gm = float(np.exp(np.mean([np.log(r["views_per_s"]) for r in rows])))
     print(json.dumps({"metric": METRIC, "value": gm, "unit": "views/s", "n_gpus": 1, "steps": steps, "warmup": warmup,
                       "ms_per_step": float(np.mean([r["ms_per_step"] for r in rows])), "higher_is_better": True, "scaling": "weak",
@@ -397,10 +420,14 @@ def run_ours(args, wl):
         sampler.start()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
-    for i in range(args.steps):
+    for i in range(args.steps - 1):
         step(warmup + i)
+    last = step(warmup + args.steps - 1)
     ev1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     t = torch.tensor([ev0.elapsed_time(ev1)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -561,7 +588,12 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=8)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.workload == "sweep":
         if args.impl == "reference":
             print(json.dumps({"impl": "reference", "unavailable": "the sweep workload has no reference arm (use cfg2/cfg3)"}))

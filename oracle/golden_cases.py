@@ -43,7 +43,8 @@ CASES = {
 }
 
 SUBSAMPLE = 48     # pixels per item frozen for the big cases
-DENSE = 1024       # pixels per item of the dense fixtures (<case>_dense.npz) of the BASELINE-sized cases below
+DENSE = 128        # pixels per item of the dense fixtures (<case>_dense.npz) of the BASELINE-sized cases below;
+                   # sized so that each fixture stays under 1 MB
 DENSE_CASES = ("cfg2_r50_256_randn", "cfg3_r152_384")
 
 

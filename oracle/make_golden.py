@@ -62,7 +62,7 @@ def main(names=None):
         path = os.path.join(out_dir, name + ".npz")
         np.savez_compressed(path, **rec)
         print("%-22s %8.1f KB  out|max|=%.4g" % (name, os.path.getsize(path) / 1024, np.abs(r["out"]).max()))
-        if name in gc.DENSE_CASES:                              # 1024 pixels per item: T1/T3 at BASELINE shapes with real coverage
+        if name in gc.DENSE_CASES:                              # DENSE pixels per item: T1/T3 at BASELINE shapes with real coverage
             px = gc.dense_pixels(name)
             n_idx = np.arange(spec["N"])[:, None]
             yy, xx = px[..., 0], px[..., 1]

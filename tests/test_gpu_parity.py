@@ -112,7 +112,7 @@ def test_T1_golden_subsampled(name, variant):
 
 @pytest.mark.parametrize("name", DENSE)
 def test_T1_T3_dense_baseline_shapes(name, capsys):
-    """BASELINE shapes with real coverage: 1024 frozen pixels per item (25 % / 11 % of the cfg2 / cfg3 maps).
+    """BASELINE shapes with real coverage: 128 frozen pixels per item (3.1 % / 1.4 % of the cfg2 / cfg3 maps).
     T1: reference locations injected there -> out / attn within 1e-4, correspondences exact up to reference ties.
     T3 (SURVEY.md 8c): the three norms  |kernel - ref_fp32|, |kernel - oracle(fp64 locs)|, |ref_fp32 - oracle(fp64 locs)|
     on those pixels; the kernel's own geometry must be at least as close to the fp64-geometry oracle as the reference is."""

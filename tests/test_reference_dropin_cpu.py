@@ -1,63 +1,37 @@
-"""CPU (build container only): the drop-in really drops in.  The UNMODIFIED reference PoseResNet
-(/root/reference/modeling/backbones/resnet.py:257-305) is constructed with its `Epipolar` name re-bound to ours, exactly
-as INTEGRATION.md section 2 prescribes, and a state dict produced by the reference-built model loads strictly.
-Skipped where /root/reference does not exist (the GPU box)."""
-import importlib
+"""CPU: the drop-in really drops in.  INTEGRATION.md section 2 re-binds the `Epipolar` name of the reference's PoseResNet
+(modeling/backbones/resnet.py:257-305) to ours; a checkpoint of the reference-built model must then load strictly and the
+model's call (resnet.py:385-387) must find the same forward parameters.  What the reference model expects of its
+`epipolar_sampler` is frozen in tests/golden/pose_resnet_epipolar_sampler.json by oracle/make_golden_dropin.py."""
+import inspect
+import json
 import os
-import sys
-import tempfile
-import types
-import warnings
 
-import pytest
+import torch
 
-from oracle import ref_harness as rh
-
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="reference tree not present")
-
-
-def _import_reference_resnet():
-    warnings.filterwarnings("ignore")
-    _, ref_cfg = rh.load_reference()
-    import PIL
-    if not hasattr(PIL, "PILLOW_VERSION"):               # the reference targets Pillow < 7 (data/transforms/image.py:6)
-        PIL.PILLOW_VERSION = PIL.__version__
-    R = rh.REFERENCE_ROOT
-    for name, sub in (("modeling.backbones", ("modeling", "backbones")), ("data", ("data",)),
-                      ("data.transforms", ("data", "transforms")), ("utils", ("utils",))):
-        if name not in sys.modules:                      # leaf packages only: modeling/__init__.py pulls the whole model zoo
-            pkg = types.ModuleType(name)
-            pkg.__path__ = [os.path.join(R, *sub)]
-            sys.modules[name] = pkg
-    ref_cfg.FOLDER_NAME = tempfile.mkdtemp()             # resnet.py:16 opens a log file there at import time
-    return importlib.import_module("modeling.backbones.resnet"), ref_cfg
+GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pose_resnet_epipolar_sampler.json")))
 
 
 def test_epipolar_drops_into_reference_pose_resnet():
     import epipolar_transformers_b200 as epi
-    rn, ref_cfg = _import_reference_resnet()
     ours = epi.cfg_h36m_r50_256()                        # configs/epipolar/keypoint_h36m_zresidual_fixed.yaml shape
-    rh.apply_cfg(ref_cfg, ours)
-    ref_cfg.BACKBONE.BODY = "epipolarposeR-50"
-    reference_epipolar = rn.Epipolar
-    m_ref = rn.PoseResNet(rn.Bottleneck, [3, 4, 6, 3], ref_cfg)          # resnet.py:299-305 instantiates Epipolar()
-    assert type(m_ref.epipolar_sampler) is reference_epipolar
-    sd = m_ref.state_dict()
-    try:
-        rn.Epipolar = lambda *a, **k: epi.Epipolar(*a, cfg=ours, **k)    # the monkey-patch of INTEGRATION.md section 2
-        m_new = rn.PoseResNet(rn.Bottleneck, [3, 4, 6, 3], ref_cfg)
-    finally:
-        rn.Epipolar = reference_epipolar
-    assert isinstance(m_new.epipolar_sampler, epi.Epipolar)
-    assert set(m_new.state_dict()) == set(sd)                            # identical parameter / buffer names
+    m_new = epi.Epipolar(cfg=ours)
+    want = GOLD["sampler_state"]
+    assert set(m_new.state_dict()) == set(want)                          # identical parameter / buffer names
+    # a state dict shaped like the reference model's `epipolar_sampler.*` entries, with values to check the load
+    gen = torch.Generator().manual_seed(0)
+    sd = {k: (torch.randn(v["shape"], generator=gen).to(getattr(torch, v["dtype"])) if v["dtype"].startswith("float")
+              else torch.full(v["shape"], 7, dtype=getattr(torch, v["dtype"])))
+          for k, v in want.items()}
     res = m_new.load_state_dict(sd, strict=True)
     assert not res.missing_keys and not res.unexpected_keys
+    for k, v in m_new.state_dict().items():
+        assert v.dtype == sd[k].dtype and torch.equal(v, sd[k]), k
     for k in ("z.weight", "z.bias", "bn.weight", "bn.bias", "bn.running_mean", "bn.running_var"):
-        assert tuple(getattr_path(m_new.epipolar_sampler, k).shape) == tuple(sd["epipolar_sampler." + k].shape)
+        assert list(getattr_path(m_new, k).shape) == want[k]["shape"]
     # the forward signature the caller uses (resnet.py:385-387): positional feats/KRTs + camera kwargs
-    import inspect
-    params = list(inspect.signature(m_new.epipolar_sampler.forward).parameters)
+    params = list(inspect.signature(m_new.forward).parameters)
     assert params[:4] == ["feat1", "feat2", "P1", "P2"] and "camera" in params and "other_camera" in params
+    assert params == GOLD["forward_params"]
 
 
 def getattr_path(obj, path):
